@@ -5,6 +5,9 @@ loop-closure search at 64x900, on synthetic KITTI-shaped data.
   python bench.py --gpus N --steps K --warmup W            # this repo's B200 path
   python bench.py --impl reference --steps K --warmup W    # the CPU port of the reference, host cores
   (N > 1: python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...)
+  --dump-outputs DIR   also write what the last timed headline step returned (every candidate's
+                       overlap and yaw, float32 .npy) so that two builds can be compared output for
+                       output; the inputs depend only on the arguments.
 
 Headline (`value`, `e2e`): BASELINE config 2 -- one query scan through the whole hot path,
   raw cloud (124 668 pts) -> projection + normals (64x900x4) -> leg -> 1 x 1101 delta + correlation
@@ -63,7 +66,12 @@ def parse():
   ap.add_argument('--cpu-pairs', type=int, default=8, help='pairs per step in the CPU sample')
   ap.add_argument('--transport', default='auto', choices=['auto', 'symm', 'collective'])
   ap.add_argument('--no-extras', action='store_true', help='only the headline config (fast)')
-  return ap.parse_args()
+  ap.add_argument('--dump-outputs', metavar='DIR',
+                  help='write the overlaps and yaws of the last timed headline step to DIR/{overlap,yaw}.npy')
+  args = ap.parse_args()
+  if args.steps < 1:
+    ap.error('--steps must be at least 1')
+  return args
 
 
 def peaks():
@@ -334,6 +342,9 @@ def main():
   eng.check()
   gpu_ov = last['res'][0][:N_CAND].cpu().numpy() if rank == 0 else None     # rank 0's own shard of the last timed step
   gpu_yaw = last['res'][1][:N_CAND].cpu().numpy() if rank == 0 else None
+  if rank == 0 and args.dump_outputs:                        # every rank's candidates, in bank order
+    dump = {'overlap': last['res'][0].cpu().numpy().astype(np.float32),
+            'yaw': last['res'][1].cpu().numpy().astype(np.float32)}
   last_q = (args.steps - 1) % n_q if args.steps else 0
   # ---- timed region 2: end to end through the host-buffer entry point
   ms_e2e = timed(step_e2e, args.steps, args.warmup)
@@ -413,6 +424,10 @@ def main():
         'clocks': clocks,
     }
     line.update(extras)
+    if args.dump_outputs:
+      os.makedirs(args.dump_outputs, exist_ok=True)
+      for name, a in dump.items():
+        np.save(os.path.join(args.dump_outputs, name + '.npy'), a)
     print(json.dumps(line))
   if world > 1:
     dist.barrier()

@@ -10,8 +10,8 @@ projection.py  NumPy restatement of ``src/utils/utils.py:59-186`` (range_project
                gen_normal_map) and the cue drivers ``src/utils/gen_*_data.py``.
                PARITY PINNED: bit-exact against the reference's shipped fixtures
                (``data/scans/*.bin`` -> ``data/preprocess_data_demo/**.npy``) and against the
-               reference's own functions imported from /root/reference (tests/test_oracle_*.py,
-               tools/make_golden.py).
+               outputs of the reference's own functions stored under tests/golden/
+               (tests/test_oracle_*.py, tools/make_golden.py, tools/make_golden_reference.py).
 network.py     torch-CPU restatement of the leg (``generateNet.py:119-219``), the delta head
                (``generateNet.py:15-116``), the circular padding (``RangePadding2D.py:31-41``),
                the correlation head (``NormalizedCorrelation2D.py:43-109``) and the readout

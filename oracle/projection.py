@@ -1,10 +1,9 @@
 """NumPy oracle for the preprocessing stage (TEST INFRASTRUCTURE, see oracle/__init__.py).
 
 Restates, operation by operation and in float32, what the reference computes in
-``/root/reference/src/utils/utils.py`` and the ``gen_*_data.py`` drivers.  Parity is PINNED:
+its ``src/utils/utils.py`` and the ``gen_*_data.py`` drivers.  Parity is PINNED:
 ``tests/test_oracle_projection.py`` checks every function here bit-for-bit against the golden
-vectors generated from the reference (``tools/make_golden.py``) and, when /root/reference is
-present, against the reference's functions imported live.
+vectors generated from the reference (``tools/make_golden.py``, ``tools/make_golden_reference.py``).
 
 Two places where the reference's result depends on the host's NumPy build are given a canonical,
 host-independent definition here (and the CUDA kernels implement the same definition):

@@ -9,7 +9,6 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if ROOT not in sys.path:
   sys.path.insert(0, ROOT)
 GOLDEN = os.path.join(ROOT, 'tests', 'golden')
-REFERENCE = '/root/reference'
 
 
 def pytest_configure(config):
@@ -33,6 +32,13 @@ def pytest_collection_modifyitems(config, items):
 @pytest.fixture(scope='session')
 def manifest():
   with open(os.path.join(GOLDEN, 'MANIFEST.json')) as f:
+    return json.load(f)
+
+
+@pytest.fixture(scope='session')
+def reference_outputs():
+  """What the reference computed on the parity inputs (tools/make_golden_reference.py)."""
+  with open(os.path.join(GOLDEN, 'reference_outputs.json')) as f:
     return json.load(f)
 
 

@@ -1,6 +1,7 @@
 """Oracle of the ground-truth overlap / yaw generator vs the golden vectors produced by the
-reference's own ``com_overlap_yaw`` (tools/make_golden_gt.py), and live against the reference
-when /root/reference is present."""
+reference's own ``com_overlap_yaw`` (tools/make_golden_gt.py) and ``range_projection``
+(tools/make_golden_reference.py)."""
+import hashlib
 import io
 import os
 import sys
@@ -16,7 +17,6 @@ from make_golden_gt import gt_test_clouds  # noqa: E402
 from oracle import gt as G  # noqa: E402
 
 GOLDEN = os.path.join(ROOT, 'tests', 'golden')
-REF_UTILS = '/root/reference/src/utils'
 
 
 @pytest.fixture(scope='module')
@@ -56,13 +56,13 @@ def test_range_image_is_float32_of_float64_minimum():
   assert np.all(img[img <= 0] == -1)
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_UTILS), reason='reference not mounted')
-def test_live_reference_range_image(fixture):
+def test_live_reference_range_image(fixture, reference_outputs):
+  """The reference's range_projection of float64 clouds, stored as hashes (tools/make_golden_reference.py)."""
   clouds, poses, _ = fixture
-  sys.path.insert(0, REF_UTILS)
-  import utils as ref_utils
-  for c, T in zip(clouds[:3], poses[:3]):
+  for c, T, want in zip(clouds[:3], poses[:3], reference_outputs['gt_range_frame2']):
     v = G.homogeneous_points(c)
     v = np.linalg.inv(poses[2]).dot(T.dot(v.T)).T
-    want, _, _, _ = ref_utils.range_projection(v)
-    assert np.array_equal(G.range_image_f64(v), want)
+    img = G.range_image_f64(v)
+    assert img.dtype == np.float32 and img.shape == (64, 900)
+    assert int((img > 0).sum()) == want['filled']
+    assert hashlib.sha256(np.ascontiguousarray(img).tobytes()).hexdigest() == want['range_sha']
