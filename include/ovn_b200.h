@@ -232,6 +232,32 @@ int ovn_get_feature_center(ovn_handle* h, float* h_mu /* [128] */, int32_t* is_s
  * explicit, so that handles on different GPUs (a sharded bank) produce bit-identical results. */
 int ovn_calibrate(ovn_handle* h, const float* d_volume, void* stream);
 
+/* ---- overlap-head training on a frozen leg (training.py with legsType 360OutputkLegsFixed,
+ * generateNet.py:222-324).  The forward and all gradients but dW1 run in fp32; dW1 runs in fp32 on
+ * precision fp32 handles and on tensor cores (fp16 operands, fp32 accumulation) on f16_tc handles.
+ * ovn_heads_backward: for pairs LEFT = d_bank[d_left[p]], RIGHT = d_bank[d_right[p]]
+ * (ImagePairOverlapOrientationSequence.py:100-112) runs both heads, the losses
+ *   d_losses[0] = 5 * L_ov + L_or, d_losses[1] = L_ov (my_sigmoid_loss, training.py:71-83),
+ *   d_losses[2] = L_or (my_entropy, training.py:86-92: target bin d_yaw_bin_gt[p] carries
+ *   d_overlap_gt[p] and counts as positive when > min_overlap_for_angle; pos_weight = 360)
+ * and OVERWRITES the gradients of c_conv1..3 and overlap_output (L_or has none) held by the handle.
+ * n_pairs <= max_batch_pairs (else OVN_ERR_CAPACITY).  Indices and yaw bins are range-checked on the
+ * device like ovn_heads_forward (deferred error, ovn_check; the losses are NaN).  The training
+ * workspace and the Adagrad state are allocated on the first call. */
+int ovn_heads_backward(ovn_handle* h, const float* d_bank, int64_t bank_size,
+                       const int32_t* d_left_idx, const int32_t* d_right_idx, int32_t n_pairs,
+                       const float* d_overlap_gt, const int32_t* d_yaw_bin_gt, float min_overlap_for_angle,
+                       float* d_losses /* [3] */, void* stream);
+/* Gradient of a head layer (c_conv1..3, overlap_output) in Keras layout; synchronises the device. */
+int ovn_get_gradient(ovn_handle* h, const char* layer_name, float* h_kernel, float* h_bias);
+/* Keras 2.1.5 Adagrad (training.py:253) on the device fp32 weights of the four head layers:
+ * a += g^2; w -= lr * g / (sqrt(a) + 1e-7).  Accumulators start at zero and are reset by
+ * ovn_set_weights.  Afterwards the inference entry points refuse (OVN_ERR_WEIGHTS) until
+ * ovn_finalize_weights repacks from the trained weights (and re-calibrates the centres on next use). */
+int ovn_adagrad_step(ovn_handle* h, float lr, void* stream);
+/* Current weights of any layer in Keras layout (trained head weights included); synchronises. */
+int ovn_get_weights(ovn_handle* h, const char* layer_name, float* h_kernel, float* h_bias);
+
 /* ---- host-buffer convenience entry points (what a non-CUDA caller binds; bench.py e2e) ------ */
 /* Raw clouds on the host -> feature volumes on the host. */
 int ovn_encode_clouds_host(ovn_handle* h, const float* h_points, const int64_t* h_offsets,

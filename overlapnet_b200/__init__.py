@@ -15,6 +15,9 @@ def __getattr__(name):
   if name == 'Infer':
     from .infer import Infer
     return Infer
+  if name == 'Trainer':
+    from .train import Trainer
+    return Trainer
   if name == 'Engine':
     from .engine import Engine
     return Engine

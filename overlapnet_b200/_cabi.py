@@ -20,6 +20,7 @@ SYMBOLS = [
     'ovn_leg_forward', 'ovn_heads_forward', 'ovn_heads_1vsN', 'ovn_bank_prepare', 'ovn_bank_release', 'ovn_encode_clouds_host',
     'ovn_query_cloud_vs_bank_host', 'ovn_check', 'ovn_set_feature_center', 'ovn_get_feature_center',
     'ovn_heads_rows_vs_bank', 'ovn_calibrate', 'ovn_peer_signal', 'ovn_peer_wait',
+    'ovn_heads_backward', 'ovn_get_gradient', 'ovn_adagrad_step', 'ovn_get_weights',
 ]
 
 
@@ -92,6 +93,10 @@ def lib():
   L.ovn_calibrate.argtypes = [vp, vp, vp]
   L.ovn_peer_signal.argtypes = [vp, vp, i32, i32, vp]
   L.ovn_peer_wait.argtypes = [vp, vp, i32, i32, i32, vp]
+  L.ovn_heads_backward.argtypes = [vp, vp, i64, vp, vp, i32, vp, vp, f32, vp, vp]
+  L.ovn_get_gradient.argtypes = [vp, C.c_char_p, vp, vp]
+  L.ovn_adagrad_step.argtypes = [vp, f32, vp]
+  L.ovn_get_weights.argtypes = [vp, C.c_char_p, vp, vp]
   L.ovn_encode_clouds_host.argtypes = [vp, vp, vp, i32, vp]
   L.ovn_query_cloud_vs_bank_host.argtypes = [vp, vp, i64, vp, i64, vp, i32, vp, vp, vp]
   _lib = L

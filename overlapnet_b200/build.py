@@ -9,7 +9,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, 'csrc')
 LIB = os.path.join(HERE, 'libovn_b200.so')
 PROBE = os.path.join(HERE, 'umma_probe')
-SOURCES = ['api.cu', 'projection.cu', 'gt_overlap.cu', 'network_fp32.cu', 'network_tc.cu']
+SOURCES = ['api.cu', 'projection.cu', 'gt_overlap.cu', 'network_fp32.cu', 'network_tc.cu', 'train.cu']
 NVCC_FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-lineinfo', '-O3', '-std=c++17',
               '-Xcompiler', '-fPIC'] + os.environ.get('OVN_NVCC_EXTRA', '').split()      # e.g. -DOVN_K4_ROT=0 for A/B timing
 

@@ -85,6 +85,7 @@ int check_device_error(ovn_handle* h, cudaStream_t s) {
   if (e == kErrBadIndex) OVN_SET_ERR(h, OVN_ERR_INVALID_ARG, "a pair / candidate index is outside [0, bank_size)");
   if (e == kErrRowNotPrepared)
     OVN_SET_ERR(h, OVN_ERR_INVALID_ARG, "resident bank: an indexed row was never passed to ovn_bank_prepare");
+  if (e == kErrBadYawBin) OVN_SET_ERR(h, OVN_ERR_INVALID_ARG, "a yaw-bin target is outside [0, leg_output_width)");
   if (e == 950) OVN_SET_ERR(h, OVN_ERR_CUDA, "ovn_peer_wait timed out: a peer rank never signalled");
   OVN_SET_ERR(h, OVN_ERR_CUDA, "tensor-core pipeline barrier timed out (code %d); outputs of the call are poisoned (NaN / INT32_MIN)", e);
 }
@@ -241,6 +242,7 @@ int ovn_create(const ovn_config* cfg, ovn_handle** out) {
   CREATE_CUDA(cudaMalloc(&h->d_err, sizeof(int)));
   CREATE_CUDA(cudaMemset(h->d_err, 0, sizeof(int)));
   CREATE_CUDA(cudaEventCreateWithFlags(&h->ev_bank, cudaEventDisableTiming));
+  CREATE_CUDA(cudaEventCreateWithFlags(&h->ev_train, cudaEventDisableTiming));
   // pinned staging of the host entry points: [err int, pad][offsets 2 x i64][cand idx][overlap][yaw]
   h->cap_pinned = 64 + (int64_t)c.max_batch_pairs * 12;
   CREATE_CUDA(cudaHostAlloc(&h->h_pinned, (size_t)h->cap_pinned, cudaHostAllocDefault));
@@ -261,6 +263,7 @@ int ovn_destroy(ovn_handle* h) {
   if (!h) return OVN_OK;
   DeviceGuard guard(h);
   tc_free(h);
+  train_free(h);
   for (auto& p : h->d_w) if (p) cudaFree(p);
   for (auto& p : h->d_b) if (p) cudaFree(p);
   for (auto& p : h->d_w16) if (p) cudaFree(p);
@@ -270,6 +273,7 @@ int ovn_destroy(ovn_handle* h) {
   for (void* b : bufs) if (b) cudaFree(b);
   if (h->h_pinned) cudaFreeHost(h->h_pinned);
   if (h->ev_bank) cudaEventDestroy(h->ev_bank);
+  if (h->ev_train) cudaEventDestroy(h->ev_train);
   if (h->own_stream) cudaStreamDestroy(h->own_stream);
   for (auto& v : h->prof_ev) for (cudaEvent_t e : v) cudaEventDestroy(e);
   delete h;
@@ -317,6 +321,24 @@ static const ConvSpec* find_layer(const ovn_handle* h, const char* name, int* sl
   return nullptr;
 }
 
+static const char* kHeadNames[4] = {"c_conv1", "c_conv2", "c_conv3", "overlap_output"};
+
+// After Adagrad steps the device fp32 head weights are the newest copy: bring them back into host_w,
+// which ovn_finalize_weights packs from.
+static int sync_trained_weights(ovn_handle* h) {
+  if (!h->weights_trained) return OVN_OK;
+  OVN_CUDA(h, cudaEventSynchronize(h->ev_train));
+  for (int l = 0; l < 4; ++l) {
+    LayerWeights& w = h->host_w[kHeadNames[l]];
+    OVN_CUDA(h, cudaMemcpy(w.kernel.data(), h->d_w[kMaxLegLayers + l], w.kernel.size() * sizeof(float),
+                           cudaMemcpyDeviceToHost));
+    OVN_CUDA(h, cudaMemcpy(w.bias.data(), h->d_b[kMaxLegLayers + l], w.bias.size() * sizeof(float),
+                           cudaMemcpyDeviceToHost));
+  }
+  h->weights_trained = false;
+  return OVN_OK;
+}
+
 int ovn_set_weights(ovn_handle* h, const char* name, const float* k, const int64_t* dims, int32_t ndim,
                     const float* bias, int64_t bias_len) {
   if (!h) return OVN_ERR_INVALID_ARG;
@@ -345,6 +367,11 @@ int ovn_set_weights(ovn_handle* h, const char* name, const float* k, const int64
                   (long long)dims[i], (long long)expect[i]);
     total *= dims[i];
   }
+  {
+    int rc = sync_trained_weights(h);
+    if (rc != OVN_OK) return rc;
+  }
+  train_reset_optimizer(h);                 // new weights start a new Adagrad run
   LayerWeights& w = h->host_w[name];
   w.kernel.assign(k, k + total);
   w.dims.assign(dims, dims + ndim);
@@ -368,6 +395,10 @@ int ovn_finalize_weights(ovn_handle* h) {
   if (!h) return OVN_ERR_INVALID_ARG;
   DeviceGuard guard(h);
   if (!h->net_ok) OVN_SET_ERR(h, OVN_ERR_BAD_CONFIG, "ovn_finalize_weights: %s", h->net_error.c_str());
+  {
+    int rc = sync_trained_weights(h);
+    if (rc != OVN_OK) return rc;
+  }
   for (int l = 0; l < h->n_leg; ++l) {
     auto it = h->host_w.find(h->leg[l].name);
     if (it == h->host_w.end() || !it->second.set)
@@ -375,11 +406,10 @@ int ovn_finalize_weights(ovn_handle* h) {
     int rc = upload(h, l, it->second);
     if (rc != OVN_OK) return rc;
   }
-  const char* hn[4] = {"c_conv1", "c_conv2", "c_conv3", "overlap_output"};
   for (int l = 0; l < 4; ++l) {
-    auto it = h->host_w.find(hn[l]);
+    auto it = h->host_w.find(kHeadNames[l]);
     if (it == h->host_w.end() || !it->second.set)
-      OVN_SET_ERR(h, OVN_ERR_WEIGHTS, "ovn_finalize_weights: layer %s has no weights", hn[l]);
+      OVN_SET_ERR(h, OVN_ERR_WEIGHTS, "ovn_finalize_weights: layer %s has no weights", kHeadNames[l]);
     int rc = upload(h, kMaxLegLayers + l, it->second);
     if (rc != OVN_OK) return rc;
   }
@@ -491,6 +521,8 @@ static int heads_dispatch(ovn_handle* h, const float* d_bank, int64_t bank_size,
                           float* d_corr, cudaStream_t s) {
   if (!h->net_ok) OVN_SET_ERR(h, OVN_ERR_BAD_CONFIG, "heads: %s", h->net_error.c_str());
   if (!h->weights_ready) OVN_SET_ERR(h, OVN_ERR_WEIGHTS, "heads: weights not finalised");
+  if (h->weights_trained)
+    OVN_SET_ERR(h, OVN_ERR_WEIGHTS, "heads: weights changed by training; call ovn_finalize_weights");
   if (bank_size <= 0) OVN_SET_ERR(h, OVN_ERR_INVALID_ARG, "heads: bank_size must be positive");
   // Every index list is bounds-checked on the device (no host sync): out-of-range entries are clamped,
   // the error flag is raised, the finalize kernels poison the outputs and the next synchronising
@@ -644,6 +676,72 @@ int ovn_bank_release(ovn_handle* h, const float* d_bank) {
   DeviceGuard guard(h);
   if (h->cfg.precision != OVN_PREC_F16_TC) return OVN_OK;
   return tc_bank_release(h, d_bank);
+}
+
+// ---- head training on a frozen leg (train.cu) -------------------------------------------------------
+static int head_layer_index(const char* name) {
+  for (int l = 0; l < 4; ++l)
+    if (name && strcmp(name, kHeadNames[l]) == 0) return l;
+  return -1;
+}
+
+int ovn_heads_backward(ovn_handle* h, const float* d_bank, int64_t bank_size, const int32_t* d_left,
+                       const int32_t* d_right, int32_t n_pairs, const float* d_overlap_gt, const int32_t* d_yaw_bin_gt,
+                       float min_overlap_for_angle, float* d_losses, void* stream) {
+  if (!h) return OVN_ERR_INVALID_ARG;
+  DeviceGuard guard(h);
+  REQUIRE(h, n_pairs > 0 && bank_size > 0, "n_pairs and bank_size must be positive");
+  REQUIRE(h, d_bank && d_left && d_right && d_overlap_gt && d_yaw_bin_gt && d_losses, "NULL pointer");
+  if (!h->net_ok) OVN_SET_ERR(h, OVN_ERR_BAD_CONFIG, "ovn_heads_backward: %s", h->net_error.c_str());
+  if (!h->weights_ready) OVN_SET_ERR(h, OVN_ERR_WEIGHTS, "ovn_heads_backward: weights not finalised");
+  if (n_pairs > h->cfg.max_batch_pairs)
+    OVN_SET_ERR(h, OVN_ERR_CAPACITY, "ovn_heads_backward: n_pairs=%d exceeds max_batch_pairs=%d", n_pairs,
+                h->cfg.max_batch_pairs);
+  int rc = train_heads_backward(h, d_bank, bank_size, d_left, d_right, n_pairs, d_overlap_gt, d_yaw_bin_gt,
+                                min_overlap_for_angle, d_losses, (cudaStream_t)stream);
+  if (rc == OVN_OK) OVN_CUDA(h, cudaEventRecord(h->ev_train, (cudaStream_t)stream));
+  return rc;
+}
+
+int ovn_get_gradient(ovn_handle* h, const char* layer_name, float* h_kernel, float* h_bias) {
+  if (!h) return OVN_ERR_INVALID_ARG;
+  DeviceGuard guard(h);
+  const int l = head_layer_index(layer_name);
+  if (l < 0) OVN_SET_ERR(h, OVN_ERR_WEIGHTS, "ovn_get_gradient: '%s' is not a trained head layer",
+                         layer_name ? layer_name : "(null)");
+  return train_get_gradient(h, l, h_kernel, h_bias);
+}
+
+int ovn_adagrad_step(ovn_handle* h, float lr, void* stream) {
+  if (!h) return OVN_ERR_INVALID_ARG;
+  DeviceGuard guard(h);
+  REQUIRE(h, isfinite(lr) && lr >= 0.f, "learning rate must be finite and non-negative");
+  int rc = train_adagrad_step(h, lr, (cudaStream_t)stream);
+  if (rc == OVN_OK) {
+    h->weights_trained = true;
+    OVN_CUDA(h, cudaEventRecord(h->ev_train, (cudaStream_t)stream));
+  }
+  return rc;
+}
+
+int ovn_get_weights(ovn_handle* h, const char* layer_name, float* h_kernel, float* h_bias) {
+  if (!h) return OVN_ERR_INVALID_ARG;
+  DeviceGuard guard(h);
+  REQUIRE(h, layer_name && h_kernel && h_bias, "NULL pointer");
+  auto it = h->host_w.find(layer_name);
+  if (it == h->host_w.end() || !it->second.set)
+    OVN_SET_ERR(h, OVN_ERR_WEIGHTS, "ovn_get_weights: layer '%s' has no weights", layer_name);
+  const LayerWeights& w = it->second;
+  const int l = head_layer_index(layer_name);
+  if (l >= 0 && h->weights_trained) {        // the device master copy is newer than host_w
+    OVN_CUDA(h, cudaEventSynchronize(h->ev_train));
+    OVN_CUDA(h, cudaMemcpy(h_kernel, h->d_w[kMaxLegLayers + l], w.kernel.size() * sizeof(float), cudaMemcpyDeviceToHost));
+    OVN_CUDA(h, cudaMemcpy(h_bias, h->d_b[kMaxLegLayers + l], w.bias.size() * sizeof(float), cudaMemcpyDeviceToHost));
+    return OVN_OK;
+  }
+  memcpy(h_kernel, w.kernel.data(), w.kernel.size() * sizeof(float));
+  memcpy(h_bias, w.bias.data(), w.bias.size() * sizeof(float));
+  return OVN_OK;
 }
 
 // ---- host-buffer entry points ---------------------------------------------------------------------

@@ -32,7 +32,7 @@ struct LayerWeights {
 
 }  // namespace ovn
 
-namespace ovn { struct TcState; }
+namespace ovn { struct TcState; struct TrainState; }
 
 struct ovn_handle {
   ovn_config cfg;
@@ -89,6 +89,9 @@ struct ovn_handle {
   bool profiling = false;
   std::vector<cudaEvent_t> prof_ev[ovn::kProfKinds];   // start/stop pairs, in launch order
   ovn::TcState* tc = nullptr;              // tensor-core path state (network_tc.cu)
+  ovn::TrainState* tr = nullptr;           // head-training buffers and Adagrad state (train.cu), allocated on first use
+  bool weights_trained = false;
+  cudaEvent_t ev_train = nullptr;          // recorded after each training call: read-backs wait on it, not on the device            // an Adagrad step changed the device head weights: packs are stale
 };
 
 #define OVN_SET_ERR(h, code, ...)                                 \
@@ -134,6 +137,7 @@ struct DeviceGuard {
 // error codes written to ovn_handle::d_err by kernels
 constexpr int kErrBadIndex = 900;        // a pair / candidate index outside [0, bank_size)
 constexpr int kErrRowNotPrepared = 901;  // resident bank: the row was never passed to ovn_bank_prepare
+constexpr int kErrBadYawBin = 902;       // training: a yaw-bin target outside [0, leg_output_width)
 
 // RAII-free profiling helpers: record an event on `s` before / after a launch when enabled
 inline void prof_mark(ovn_handle* h, int kind, cudaStream_t s) {
@@ -182,6 +186,14 @@ void tc_free(ovn_handle* h);
 int tc_set_center(ovn_handle* h, const float* h_mu);
 int tc_get_center(ovn_handle* h, float* h_mu, int32_t* is_set);
 int tc_calibrate(ovn_handle* h, const float* d_volume, cudaStream_t s);
+// head training (train.cu)
+int train_heads_backward(ovn_handle* h, const float* d_bank, int64_t bank_size, const int32_t* d_left,
+                         const int32_t* d_right, int n, const float* d_ov_gt, const int32_t* d_bin_gt,
+                         float min_ov_angle, float* d_losses, cudaStream_t s);
+int train_adagrad_step(ovn_handle* h, float lr, cudaStream_t s);
+int train_get_gradient(ovn_handle* h, int layer, float* h_kernel, float* h_bias);
+void train_reset_optimizer(ovn_handle* h);
+void train_free(ovn_handle* h);
 // bounds-checked copies of index lists (d_idx_san): out-of-range entries are clamped and flagged in d_err
 int sanitize_indices(ovn_handle* h, const int32_t* d_in, int n, int64_t limit, int code, int32_t* d_out, cudaStream_t s);
 // read (and clear) the device error flag after the caller has synchronised `s`; maps it to a status

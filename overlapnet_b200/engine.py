@@ -59,6 +59,7 @@ class Engine:
     cfg.max_batch_scans = int(max_batch_scans)
     cfg.max_batch_pairs = int(max_batch_pairs)
     self.cfg = cfg
+    self._model = model
     self.precision = precision
     self.H, self.W = proj_H, proj_W
     self._h = C.c_void_p(0)
@@ -304,6 +305,54 @@ class Engine:
 
   def bank_release(self, bank=None):
     check(self._h, lib().ovn_bank_release(self._h, _ptr(bank)), 'ovn_bank_release')
+
+  # ---- overlap-head training on a frozen leg (precision fp32) ---------------------------------
+  HEAD_LAYERS = ('c_conv1', 'c_conv2', 'c_conv3', 'overlap_output')
+
+  def heads_backward(self, bank, left_idx, right_idx, overlap_gt, yaw_bin_gt, min_overlap_for_angle=0.7):
+    """ovn_heads_backward: losses and head gradients of one batch (LEFT = bank[left_idx], RIGHT =
+    bank[right_idx]).  Returns a float32 cuda tensor [3] = (5 L_ov + L_or, L_ov, L_or); the gradients
+    stay in the handle (``gradients()``, ``adagrad_step``)."""
+    n = left_idx.numel()
+    dev = self.device
+    li = left_idx.to(device=dev, dtype=torch.int32).contiguous()
+    ri = right_idx.to(device=dev, dtype=torch.int32).contiguous()
+    ov = torch.as_tensor(overlap_gt).to(device=dev, dtype=torch.float32).contiguous()
+    yb = torch.as_tensor(yaw_bin_gt).to(device=dev, dtype=torch.int32).contiguous()
+    losses = torch.empty((3,), dtype=torch.float32, device=dev)
+    check(self._h, lib().ovn_heads_backward(self._h, _ptr(bank), int(bank.shape[0]), _ptr(li), _ptr(ri), n, _ptr(ov),
+                                           _ptr(yb), float(min_overlap_for_angle), _ptr(losses), self._stream()),
+          'ovn_heads_backward')
+    return losses
+
+  def _layer_arrays(self, fn, what, names=None):
+    from .weights import layer_shapes
+    shapes = layer_shapes(self.C, self._model, self.H, self.W)
+    out = {}
+    for name in (names or list(shapes)):
+      ks, bs = shapes[name]
+      k, b = np.empty(ks, np.float32), np.empty(bs, np.float32)
+      check(self._h, fn(self._h, name.encode(), k.ctypes.data_as(C.c_void_p), b.ctypes.data_as(C.c_void_p)),
+            '%s(%s)' % (what, name))
+      out[name] = (k, b)
+    return out
+
+  def gradients(self):
+    """{layer: (kernel grad, bias grad)} of the head layers after the last ``heads_backward``, keyed
+    like ``weights.glorot_init``; synchronises."""
+    return self._layer_arrays(lib().ovn_get_gradient, 'ovn_get_gradient', self.HEAD_LAYERS)
+
+  def get_weights(self):
+    """{layer: (kernel, bias)} of every layer, trained head weights included; synchronises."""
+    return self._layer_arrays(lib().ovn_get_weights, 'ovn_get_weights')
+
+  def adagrad_step(self, lr):
+    """ovn_adagrad_step: one Keras Adagrad update of the head weights with the last gradients."""
+    check(self._h, lib().ovn_adagrad_step(self._h, float(lr), self._stream()), 'ovn_adagrad_step')
+
+  def finalize_weights(self):
+    """ovn_finalize_weights: repack the inference path from the (trained) weights."""
+    check(self._h, lib().ovn_finalize_weights(self._h), 'ovn_finalize_weights')
 
   # ---- host-buffer entry points (synchronous) ------------------------------------------------
   def encode_clouds_host(self, clouds):
