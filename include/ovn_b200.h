@@ -248,15 +248,37 @@ int ovn_heads_backward(ovn_handle* h, const float* d_bank, int64_t bank_size,
                        const int32_t* d_left_idx, const int32_t* d_right_idx, int32_t n_pairs,
                        const float* d_overlap_gt, const int32_t* d_yaw_bin_gt, float min_overlap_for_angle,
                        float* d_losses /* [3] */, void* stream);
-/* Gradient of a head layer (c_conv1..3, overlap_output) in Keras layout; synchronises the device. */
+/* Gradient of a head layer (c_conv1..3, overlap_output) in Keras layout; synchronises the device.  The leg
+ * layers (s_conv1..s_conv10, s_conv3a) are accepted only when the last backward call was
+ * ovn_network_backward. */
 int ovn_get_gradient(ovn_handle* h, const char* layer_name, float* h_kernel, float* h_bias);
-/* Keras 2.1.5 Adagrad (training.py:253) on the device fp32 weights of the four head layers:
+/* Keras 2.1.5 Adagrad (training.py:253) on the device fp32 weights of the layers the last backward call
+ * produced gradients for (the four head layers; after ovn_network_backward also the leg):
  * a += g^2; w -= lr * g / (sqrt(a) + 1e-7).  Accumulators start at zero and are reset by
- * ovn_set_weights.  Afterwards the inference entry points refuse (OVN_ERR_WEIGHTS) until
+ * ovn_set_weights (head and leg alike).  Afterwards the inference entry points refuse (OVN_ERR_WEIGHTS) until
  * ovn_finalize_weights repacks from the trained weights (and re-calibrates the centres on next use). */
 int ovn_adagrad_step(ovn_handle* h, float lr, void* stream);
 /* Current weights of any layer in Keras layout (trained head weights included); synchronises. */
 int ovn_get_weights(ovn_handle* h, const char* layer_name, float* h_kernel, float* h_bias);
+
+/* ---- full-network training (training.py with legsType 360OutputkLegs, generateNet.py:119-219).
+ * ovn_network_backward: the Siamese leg runs on LEFT image d_inputs[d_left_idx[p]] and RIGHT image
+ * d_inputs[d_right_idx[p]] of every pair (ImagePairOverlapOrientationSequence.py:100-112), the RIGHT image
+ * rolled by d_right_roll[p] columns first (np.roll along the width, any integer, taken modulo W; NULL = no
+ * roll).  Both heads then run on the 2n feature volumes; the losses are those of ovn_heads_backward.  The
+ * call OVERWRITES the gradients of every layer: the four head layers (bit-identical to ovn_heads_backward on
+ * the same fp32 volumes) and the 11 leg layers (each the sum over both images of every pair; L_or now has
+ * a gradient).  Everything but dW1 of c_conv1 is fp32 SIMT in both precisions; dW1 follows the precision as
+ * in ovn_heads_backward.  n_pairs <= max_batch_pairs (else OVN_ERR_CAPACITY).  Indices and yaw bins are
+ * range-checked on the device (deferred error, NaN losses).  The leg training buffers are allocated on the
+ * first call and grown to the largest n_pairs seen.  Afterwards ovn_get_gradient also accepts the leg layer
+ * names, and ovn_adagrad_step also updates the leg; after such a step ovn_leg_forward (and the host entry
+ * points built on it) refuses with OVN_ERR_WEIGHTS until ovn_finalize_weights. */
+int ovn_network_backward(ovn_handle* h, const float* d_inputs /* [n_inputs][H][W][C] */, int64_t n_inputs,
+                         const int32_t* d_left_idx, const int32_t* d_right_idx,
+                         const int32_t* d_right_roll /* [n_pairs] columns, NULL = none */, int32_t n_pairs,
+                         const float* d_overlap_gt, const int32_t* d_yaw_bin_gt, float min_overlap_for_angle,
+                         float* d_losses /* [3] */, void* stream);
 
 /* ---- host-buffer convenience entry points (what a non-CUDA caller binds; bench.py e2e) ------ */
 /* Raw clouds on the host -> feature volumes on the host. */

@@ -323,8 +323,8 @@ static const ConvSpec* find_layer(const ovn_handle* h, const char* name, int* sl
 
 static const char* kHeadNames[4] = {"c_conv1", "c_conv2", "c_conv3", "overlap_output"};
 
-// After Adagrad steps the device fp32 head weights are the newest copy: bring them back into host_w,
-// which ovn_finalize_weights packs from.
+// After Adagrad steps the device fp32 head weights (and, after full-network steps, the leg weights) are
+// the newest copy: bring them back into host_w, which ovn_finalize_weights packs from.
 static int sync_trained_weights(ovn_handle* h) {
   if (!h->weights_trained) return OVN_OK;
   OVN_CUDA(h, cudaEventSynchronize(h->ev_train));
@@ -335,7 +335,12 @@ static int sync_trained_weights(ovn_handle* h) {
     OVN_CUDA(h, cudaMemcpy(w.bias.data(), h->d_b[kMaxLegLayers + l], w.bias.size() * sizeof(float),
                            cudaMemcpyDeviceToHost));
   }
-  h->weights_trained = false;
+  for (int l = 0; h->leg_trained && l < h->n_leg; ++l) {
+    LayerWeights& w = h->host_w[h->leg[l].name];
+    OVN_CUDA(h, cudaMemcpy(w.kernel.data(), h->d_w[l], w.kernel.size() * sizeof(float), cudaMemcpyDeviceToHost));
+    OVN_CUDA(h, cudaMemcpy(w.bias.data(), h->d_b[l], w.bias.size() * sizeof(float), cudaMemcpyDeviceToHost));
+  }
+  h->weights_trained = h->leg_trained = false;
   return OVN_OK;
 }
 
@@ -504,6 +509,8 @@ int ovn_leg_forward(ovn_handle* h, const float* d_input, int32_t n_scans, float*
   REQUIRE(h, d_input && d_fv, "NULL pointer");
   if (!h->net_ok) OVN_SET_ERR(h, OVN_ERR_BAD_CONFIG, "ovn_leg_forward: %s", h->net_error.c_str());
   if (!h->weights_ready) OVN_SET_ERR(h, OVN_ERR_WEIGHTS, "ovn_leg_forward: weights not finalised");
+  if (h->leg_trained)
+    OVN_SET_ERR(h, OVN_ERR_WEIGHTS, "ovn_leg_forward: weights changed by training; call ovn_finalize_weights");
   const int Wf = h->cfg.leg_output_width;
   const size_t in_stride = (size_t)h->cfg.proj_H * h->cfg.proj_W * h->C;
   for (int s0 = 0; s0 < n_scans; s0 += h->cfg.max_batch_scans) {
@@ -678,7 +685,7 @@ int ovn_bank_release(ovn_handle* h, const float* d_bank) {
   return tc_bank_release(h, d_bank);
 }
 
-// ---- head training on a frozen leg (train.cu) -------------------------------------------------------
+// ---- training: heads on a frozen leg, and the full network (train.cu) ------------------------------
 static int head_layer_index(const char* name) {
   for (int l = 0; l < 4; ++l)
     if (name && strcmp(name, kHeadNames[l]) == 0) return l;
@@ -707,18 +714,43 @@ int ovn_get_gradient(ovn_handle* h, const char* layer_name, float* h_kernel, flo
   if (!h) return OVN_ERR_INVALID_ARG;
   DeviceGuard guard(h);
   const int l = head_layer_index(layer_name);
-  if (l < 0) OVN_SET_ERR(h, OVN_ERR_WEIGHTS, "ovn_get_gradient: '%s' is not a trained head layer",
-                         layer_name ? layer_name : "(null)");
-  return train_get_gradient(h, l, h_kernel, h_bias);
+  if (l >= 0) return train_get_gradient(h, l, h_kernel, h_bias);
+  int slot = -1;
+  if (layer_name && train_has_leg_gradients(h) && find_layer(h, layer_name, &slot) && slot < kMaxLegLayers)
+    return train_get_gradient(h, kMaxLegLayers + slot, h_kernel, h_bias);
+  OVN_SET_ERR(h, OVN_ERR_WEIGHTS, "ovn_get_gradient: '%s' is not a trained head layer%s",
+              layer_name ? layer_name : "(null)",
+              train_has_leg_gradients(h) ? " or leg layer" : " (leg gradients need ovn_network_backward)");
+}
+
+int ovn_network_backward(ovn_handle* h, const float* d_inputs, int64_t n_inputs, const int32_t* d_left,
+                         const int32_t* d_right, const int32_t* d_right_roll, int32_t n_pairs,
+                         const float* d_overlap_gt, const int32_t* d_yaw_bin_gt, float min_overlap_for_angle,
+                         float* d_losses, void* stream) {
+  if (!h) return OVN_ERR_INVALID_ARG;
+  DeviceGuard guard(h);
+  REQUIRE(h, n_pairs > 0 && n_inputs > 0, "n_pairs and n_inputs must be positive");
+  REQUIRE(h, d_inputs && d_left && d_right && d_overlap_gt && d_yaw_bin_gt && d_losses, "NULL pointer");
+  if (!h->net_ok) OVN_SET_ERR(h, OVN_ERR_BAD_CONFIG, "ovn_network_backward: %s", h->net_error.c_str());
+  if (!h->weights_ready) OVN_SET_ERR(h, OVN_ERR_WEIGHTS, "ovn_network_backward: weights not finalised");
+  if (n_pairs > h->cfg.max_batch_pairs)
+    OVN_SET_ERR(h, OVN_ERR_CAPACITY, "ovn_network_backward: n_pairs=%d exceeds max_batch_pairs=%d", n_pairs,
+                h->cfg.max_batch_pairs);
+  int rc = train_network_backward(h, d_inputs, n_inputs, d_left, d_right, d_right_roll, n_pairs, d_overlap_gt,
+                                  d_yaw_bin_gt, min_overlap_for_angle, d_losses, (cudaStream_t)stream);
+  if (rc == OVN_OK) OVN_CUDA(h, cudaEventRecord(h->ev_train, (cudaStream_t)stream));
+  return rc;
 }
 
 int ovn_adagrad_step(ovn_handle* h, float lr, void* stream) {
   if (!h) return OVN_ERR_INVALID_ARG;
   DeviceGuard guard(h);
   REQUIRE(h, isfinite(lr) && lr >= 0.f, "learning rate must be finite and non-negative");
-  int rc = train_adagrad_step(h, lr, (cudaStream_t)stream);
+  bool leg_changed = false;
+  int rc = train_adagrad_step(h, lr, (cudaStream_t)stream, &leg_changed);
   if (rc == OVN_OK) {
     h->weights_trained = true;
+    if (leg_changed) h->leg_trained = true;
     OVN_CUDA(h, cudaEventRecord(h->ev_train, (cudaStream_t)stream));
   }
   return rc;
@@ -733,10 +765,12 @@ int ovn_get_weights(ovn_handle* h, const char* layer_name, float* h_kernel, floa
     OVN_SET_ERR(h, OVN_ERR_WEIGHTS, "ovn_get_weights: layer '%s' has no weights", layer_name);
   const LayerWeights& w = it->second;
   const int l = head_layer_index(layer_name);
-  if (l >= 0 && h->weights_trained) {        // the device master copy is newer than host_w
+  int slot = l >= 0 ? kMaxLegLayers + l : -1;
+  if (l < 0 && h->leg_trained) find_layer(h, layer_name, &slot);
+  if (slot >= 0 && h->weights_trained) {     // the device master copy is newer than host_w
     OVN_CUDA(h, cudaEventSynchronize(h->ev_train));
-    OVN_CUDA(h, cudaMemcpy(h_kernel, h->d_w[kMaxLegLayers + l], w.kernel.size() * sizeof(float), cudaMemcpyDeviceToHost));
-    OVN_CUDA(h, cudaMemcpy(h_bias, h->d_b[kMaxLegLayers + l], w.bias.size() * sizeof(float), cudaMemcpyDeviceToHost));
+    OVN_CUDA(h, cudaMemcpy(h_kernel, h->d_w[slot], w.kernel.size() * sizeof(float), cudaMemcpyDeviceToHost));
+    OVN_CUDA(h, cudaMemcpy(h_bias, h->d_b[slot], w.bias.size() * sizeof(float), cudaMemcpyDeviceToHost));
     return OVN_OK;
   }
   memcpy(h_kernel, w.kernel.data(), w.kernel.size() * sizeof(float));

@@ -91,7 +91,8 @@ struct ovn_handle {
   ovn::TcState* tc = nullptr;              // tensor-core path state (network_tc.cu)
   ovn::TrainState* tr = nullptr;           // head-training buffers and Adagrad state (train.cu), allocated on first use
   bool weights_trained = false;
-  cudaEvent_t ev_train = nullptr;          // recorded after each training call: read-backs wait on it, not on the device            // an Adagrad step changed the device head weights: packs are stale
+  bool leg_trained = false;                // an Adagrad step changed the device leg weights: ovn_leg_forward refuses
+  cudaEvent_t ev_train = nullptr;         // recorded after each training call: read-backs wait on it, not on the device            // an Adagrad step changed the device head weights: packs are stale
 };
 
 #define OVN_SET_ERR(h, code, ...)                                 \
@@ -190,7 +191,11 @@ int tc_calibrate(ovn_handle* h, const float* d_volume, cudaStream_t s);
 int train_heads_backward(ovn_handle* h, const float* d_bank, int64_t bank_size, const int32_t* d_left,
                          const int32_t* d_right, int n, const float* d_ov_gt, const int32_t* d_bin_gt,
                          float min_ov_angle, float* d_losses, cudaStream_t s);
-int train_adagrad_step(ovn_handle* h, float lr, cudaStream_t s);
+int train_network_backward(ovn_handle* h, const float* d_inputs, int64_t n_inputs, const int32_t* d_left,
+                           const int32_t* d_right, const int32_t* d_roll, int n, const float* d_ov_gt,
+                           const int32_t* d_bin_gt, float min_ov_angle, float* d_losses, cudaStream_t s);
+int train_adagrad_step(ovn_handle* h, float lr, cudaStream_t s, bool* leg_changed);
+bool train_has_leg_gradients(const ovn_handle* h);
 int train_get_gradient(ovn_handle* h, int layer, float* h_kernel, float* h_bias);
 void train_reset_optimizer(ovn_handle* h);
 void train_free(ovn_handle* h);

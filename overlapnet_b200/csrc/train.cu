@@ -1,6 +1,7 @@
-// train.cu -- training of the overlap head on a frozen leg (the `360OutputkLegsFixed` leg of
-// generateNet.py:222-324, fitted by training.py): forward pass with saved activations, the two
-// losses, the gradients of c_conv1..3 and overlap_output, and the Keras Adagrad update.
+// train.cu -- training (training.py): the overlap head on a frozen leg (the `360OutputkLegsFixed` leg of
+// generateNet.py:222-324; ovn_heads_backward) and the full network (`360OutputkLegs`, :119-219;
+// ovn_network_backward): forward passes with saved activations, the two losses, the gradients of the head
+// layers and, for the full network, of the feature volumes and the 11 leg layers, and the Keras Adagrad update.
 //
 // The forward pass and all gradients except dW1 are fp32 SIMT; dW1 is fp32 SIMT for precision fp32 and
 // the tcgen05 kernel k_delta_wgrad_tc for precision f16_tc.  The SIMT parts reuse the operand functors of
@@ -18,8 +19,8 @@
 //                the bins, then over the batch                                   training.py:86-92
 //   total        5 * L_ov + 1 * L_or                                             training.py:255-257
 //   Adagrad      a += g^2; p -= lr * g / (sqrt(a) + 1e-7)  (Keras 2.1.5)         training.py:253
-// The correlation head has no weights and the leg is frozen, so L_or has no gradient: it is
-// computed and reported only.
+// The correlation head has no weights: with a frozen leg L_or has no gradient and is reported only; with a
+// trainable leg it reaches the leg through the feature volumes (k_corr_logit_grad, k_dfv_finish).
 #include "simt_gemm.cuh"
 #include "umma.cuh"
 #include <math.h>
@@ -31,6 +32,7 @@ constexpr int kMaxSplits = 64;            // row splits of a weight-gradient GEM
 constexpr int kWgRows = 64;               // k_delta_wgrad_tc: rows (K) per shared-memory chunk
 constexpr int kWgSplits = 20;             // k_delta_wgrad_tc: row splits (x conv1size CTAs)
 constexpr int kErrWgradTimeout = 170;     // k_delta_wgrad_tc: MMA completion barrier timed out
+constexpr int kLegImgChunk = 64;          // images per leg GEMM launch of ovn_network_backward
 
 struct TrainState {
   int cap = 0;                            // pairs (= max_batch_pairs)
@@ -52,23 +54,46 @@ struct TrainState {
   int64_t ws_elems = 0;
   bool have_grad = false;
   bool acc_zero = true;                   // accumulators must be cleared before the next step
+  bool leg_grad = false;                  // the last backward call was ovn_network_backward
+  // ---- full-network training (ovn_network_backward), allocated on its first call
+  int leg_cap = 0;                        // pairs the activation buffers below hold (grown on demand)
+  float* x = nullptr;                     // [2 leg_cap][H][W][C] gathered inputs: LEFT images, then RIGHT
+  float* act[kMaxLegLayers] = {};         // [2 leg_cap][h_out][w_out][cout] saved leg activations
+  float* g[2] = {};                       // [2 leg_cap][max act] data-gradient ping-pong; g[0] starts as dFV
+  float* dlp = nullptr;                   // [leg_cap][nb][Wf][128] per-jb partials of dL from the overlap head
+  float* gcorr = nullptr;                 // [leg_cap][Wf] d(loss)/d(correlation logits)
+  int32_t* ident = nullptr;               // [2][leg_cap] head indices into the trained volumes: p, n + p
+  int64_t max_act = 0;                    // floats per image of the largest leg activation
+  float* wt = nullptr;                    // transposed leg kernel ([dy][dx][o][c]) of the current layer
+  float* lgk[kMaxLegLayers] = {};         // leg gradients (Keras layouts)
+  float* lgb[kMaxLegLayers] = {};
+  float* lak[kMaxLegLayers] = {};         // leg Adagrad accumulators
+  float* lab[kMaxLegLayers] = {};
+  int64_t lnk[kMaxLegLayers] = {}, lnb[kMaxLegLayers] = {};
+  bool leg_alloc = false;
+  bool leg_acc_zero = true;
 };
 
 // ---- operand functors ----------------------------------------------------------------------------
-// Data gradient of a stride-1 valid conv (c_conv3) as a GEMM over the zero-padded output gradient:
-//   A[m, k] = dY[img, y - dy, x - dx, o],  m = (img, y, x) over the INPUT grid, k = (dy, dx, o);
-// zero where (y - dy, x - dx) falls outside the Ho x Wo output.  B = the kernel as [dy][dx][o][c].
+// Data gradient of a valid conv with stride (sh, sw) as a GEMM over the zero-padded output gradient:
+//   A[m, k] = dY[img, (y - dy) / sh, (x - dx) / sw, o],  m = (img, y, x) over the INPUT grid, k = (dy, dx, o);
+// zero where (y - dy, x - dx) is not a multiple of the stride or falls outside the Ho x Wo output (input
+// rows / columns no window covers get a zero gradient).  B = the kernel as [dy][dx][o][c].  With
+// sh = sw = 1 (c_conv3) every load, and so the arithmetic, is that of the stride-free form.
 struct ConvTOperand {
   const float* dY;
   int H, W, Ho, Wo, kw, Co;
+  int sh = 1, sw = 1;
   __device__ __forceinline__ int64_t row_base(int m, int) const { return m; }
   __device__ __forceinline__ int col_off(int k) const { return k; }
   __device__ __forceinline__ float load(int64_t m64, int k, int64_t, int) const {
     const int m = (int)m64;
     const int x = m % W, t = m / W, y = t % H, img = t / H;
     const int o = k % Co, tap = k / Co, dx = tap % kw, dy = tap / kw;
-    const int yo = y - dy, xo = x - dx;
-    if (yo < 0 || yo >= Ho || xo < 0 || xo >= Wo) return 0.f;
+    const int ys = y - dy, xs = x - dx;
+    if (ys < 0 || xs < 0 || ys % sh != 0 || xs % sw != 0) return 0.f;
+    const int yo = ys / sh, xo = xs / sw;
+    if (yo >= Ho || xo >= Wo) return 0.f;
     return __ldg(dY + (((int64_t)img * Ho + yo) * Wo + xo) * Co + o);
   }
   __device__ __forceinline__ int64_t row_base2(int, int) const { return 0; }
@@ -504,14 +529,200 @@ __global__ void k_adagrad(float* __restrict__ w, const float* __restrict__ g, fl
   w[i] = w[i] - lr * gi / (sqrtf(ai) + 1e-7f);
 }
 
+// ---- full-network training: input gather, feature-volume gradients ---------------------------------
+// x[img] = inputs[left[img]] for img < n, else np.roll(inputs[right[img - n]], roll[img - n], axis=1)
+// (ImagePairOverlapOrientationSequence.py:209-212: only the RIGHT image is rolled, by whole columns).
+__global__ void k_gather_inputs(const float* __restrict__ in, const int32_t* __restrict__ left,
+                                const int32_t* __restrict__ right, const int32_t* __restrict__ roll, int n, int H,
+                                int W, int C, float* __restrict__ x) {
+  const int64_t per = (int64_t)H * W * C;
+  const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= 2 * n * per) return;
+  const int img = (int)(e / per);
+  const int64_t r = e - (int64_t)img * per;
+  const int c = (int)(r % C);
+  const int64_t yx = r / C;
+  int col = (int)(yx % W);
+  const int64_t y = yx / W;
+  int64_t src;
+  if (img < n) {
+    src = left[img];
+  } else {
+    src = right[img - n];
+    if (roll) {
+      int sh = roll[img - n] % W;                  // np.roll: out[:, x] = in[:, (x - shift) mod W]
+      if (sh < 0) sh += W;
+      col -= sh;
+      if (col < 0) col += W;
+    }
+  }
+  x[e] = __ldg(in + src * per + (y * W + col) * C + c);
+}
+
+// LEFT = p, RIGHT = n + p: the head indices into the 2n trained feature volumes
+__global__ void k_pair_ident(int32_t* __restrict__ ident, int n, int cap) {
+  const int p = blockIdx.x * blockDim.x + threadIdx.x;
+  if (p >= n) return;
+  ident[p] = p;
+  ident[cap + p] = n + p;
+}
+
+// Gradient of the yaw loss wrt the correlation logits (TF's weighted_cross_entropy_with_logits, q bins,
+// mean over bins then batch): g_p[k] = ((1 - t_k) - (1 + (q - 1) t_k) sigmoid(-x_k)) / (n q)
+__global__ void k_corr_logit_grad(const float* __restrict__ corr, const float* __restrict__ y_ov,
+                                  const int32_t* __restrict__ y_bin, float min_ov_angle, int n, int n_bins,
+                                  float* __restrict__ g) {
+  const int p = blockIdx.x;
+  const float q = (float)n_bins, yo = y_ov[p];
+  const int b = y_bin[p];
+  for (int k = threadIdx.x; k < n_bins; k += blockDim.x) {
+    const float xk = corr[(int64_t)p * n_bins + k];
+    const float tk = ((k == b ? yo : 0.f) > min_ov_angle) ? 1.f : 0.f;
+    g[(int64_t)p * n_bins + k] = ((1.f - tk) - (1.f + (q - 1.f) * tk) * sigmoidf(-xk)) / ((float)n * q);
+  }
+}
+
+// dFV from the overlap head, through c_conv1 and the delta layer (generateNet.py:15-61, 96-100):
+//   dD[i, j, c] = sum_o dO1[p, i, jb, o] W1[dj, c, o]          (j = s jb + dj)
+//   dL[i, c]   += sum_j sgn(L[i,c] - R[j,c]) dD[i, j, c],   dR[j, c] -= sum_i sgn(L[i,c] - R[j,c]) dD[i, j, c]
+// with sgn(0) = 0 (the gradient of abs in TF and torch).  dD is never stored: one block owns one (pair, jb,
+// 16-channel slice), thread (dj, c) keeps W1[dj, c, :] in registers and walks i in increasing order in
+// chunks of kDfvRows, so dR of the block's s columns is complete (fixed order) when the walk ends; the
+// per-row sum over dj runs in dj order through shared memory and lands in per-jb partials of dL, which
+// k_dfv_finish adds in jb order.  No atomics: bit-identical from call to call.
+constexpr int kDfvC = 16, kDfvRows = 16;
+__global__ void __launch_bounds__(256)
+k_dfv_overlap(const float* __restrict__ fv, const float* __restrict__ dO1, const float* __restrict__ w1, int n,
+              int Wf, int sz, int nb, float* __restrict__ dlp, float* __restrict__ dfv) {
+  __shared__ float4 s_g[kDfvRows][16];             // dO1[p, i, jb, 0..63]
+  __shared__ float s_l[kDfvRows][kDfvC];           // L[i, c0 .. c0 + 15]
+  __shared__ float s_e[kDfvRows][256];             // sgn * dD, [row][dj * kDfvC + c]
+  const int tid = threadIdx.x;
+  const int c0 = blockIdx.x * kDfvC, jb = blockIdx.y, p = blockIdx.z;
+  const int dj = tid / kDfvC, cc = tid % kDfvC;
+  const bool active = dj < sz;
+  float w[64];
+  float rv = 0.f, racc = 0.f;
+  if (active) {
+    const float4* wr = reinterpret_cast<const float4*>(w1 + ((int64_t)dj * kFeatC + c0 + cc) * 64);
+#pragma unroll
+    for (int o4 = 0; o4 < 16; ++o4) {
+      const float4 v = __ldg(wr + o4);
+      w[4 * o4] = v.x; w[4 * o4 + 1] = v.y; w[4 * o4 + 2] = v.z; w[4 * o4 + 3] = v.w;
+    }
+    rv = __ldg(fv + ((int64_t)(n + p) * Wf + sz * jb + dj) * kFeatC + c0 + cc);
+  }
+  for (int i0 = 0; i0 < Wf; i0 += kDfvRows) {
+    {
+      const int r = tid / 16, q = tid % 16;
+      const int i = i0 + r;
+      s_g[r][q] = i < Wf ? __ldg(reinterpret_cast<const float4*>(dO1 + (((int64_t)p * Wf + i) * nb + jb) * 64) + q)
+                         : make_float4(0.f, 0.f, 0.f, 0.f);
+      s_l[r][q] = i < Wf ? __ldg(fv + ((int64_t)p * Wf + i) * kFeatC + c0 + q) : 0.f;
+    }
+    __syncthreads();
+    if (active) {
+      const int rows = min(kDfvRows, Wf - i0);
+      for (int r = 0; r < rows; ++r) {
+        float d = 0.f;
+#pragma unroll
+        for (int o4 = 0; o4 < 16; ++o4) {
+          const float4 gv = s_g[r][o4];
+          d = fmaf(gv.x, w[4 * o4], d);
+          d = fmaf(gv.y, w[4 * o4 + 1], d);
+          d = fmaf(gv.z, w[4 * o4 + 2], d);
+          d = fmaf(gv.w, w[4 * o4 + 3], d);
+        }
+        const float l = s_l[r][cc];
+        const float sg = l > rv ? 1.f : (l < rv ? -1.f : 0.f);
+        const float e = sg * d;
+        s_e[r][tid] = e;
+        racc += e;
+      }
+    }
+    __syncthreads();
+    {
+      const int r = tid / kDfvC, c = tid % kDfvC;
+      if (i0 + r < Wf) {
+        float acc = 0.f;
+        for (int q = 0; q < sz; ++q) acc += s_e[r][q * kDfvC + c];
+        dlp[(((int64_t)p * nb + jb) * Wf + i0 + r) * kFeatC + c0 + c] = acc;
+      }
+    }
+  }
+  if (active) dfv[((int64_t)(n + p) * Wf + sz * jb + dj) * kFeatC + c0 + cc] = -racc;
+}
+
+// dFV of pair p's LEFT (side 0) or RIGHT (side 1) volume, rows r0 .. r0 + 7, thread = channel:
+//   correlation head (corr[k] = sum_{j,c} L[(k + j + h) mod W, c] R[j, c], h = W / 2):
+//     dL[i, c] = sum_j g[(i - j - h) mod W] R[j, c],   dR[j, c] = sum_i g[(i - j - h) mod W] L[i, c]
+//   plus the overlap head's part (LEFT: the jb partials added in jb order; RIGHT: already in dfv), then the
+//   ReLU mask of s_conv10.  Every sum runs in a fixed order.
+constexpr int kFinRows = 8;
+__global__ void __launch_bounds__(128)
+k_dfv_finish(const float* __restrict__ fv, const float* __restrict__ gcorr, const float* __restrict__ dlp, int n,
+             int Wf, int nb, float* __restrict__ dfv) {
+  extern __shared__ float s_gc[];
+  const int c = threadIdx.x, r0 = blockIdx.x * kFinRows, side = blockIdx.y, p = blockIdx.z;
+  for (int k = threadIdx.x; k < Wf; k += blockDim.x) s_gc[k] = gcorr[(int64_t)p * Wf + k];
+  __syncthreads();
+  const int self = side == 0 ? p : n + p, other = side == 0 ? n + p : p;
+  const float* ov = fv + (int64_t)other * Wf * kFeatC;
+  const int half = Wf / 2;
+  float acc[kFinRows] = {};
+  for (int u = 0; u < Wf; ++u) {
+    const float v = __ldg(ov + (int64_t)u * kFeatC + c);
+#pragma unroll
+    for (int r = 0; r < kFinRows; ++r) {
+      const int row = r0 + r;
+      int k = side == 0 ? row - u - half : u - row - half;
+      k %= Wf;
+      if (k < 0) k += Wf;
+      acc[r] = fmaf(s_gc[k], v, acc[r]);
+    }
+  }
+#pragma unroll
+  for (int r = 0; r < kFinRows; ++r) {
+    const int row = r0 + r;
+    if (row >= Wf) break;
+    const int64_t e = ((int64_t)self * Wf + row) * kFeatC + c;
+    float ovp;
+    if (side == 0) {
+      ovp = 0.f;
+      for (int jb = 0; jb < nb; ++jb) ovp += dlp[(((int64_t)p * nb + jb) * Wf + row) * kFeatC + c];
+    } else {
+      ovp = dfv[e];
+    }
+    dfv[e] = fv[e] > 0.f ? ovp + acc[r] : 0.f;
+  }
+}
+
 // ---- drivers -------------------------------------------------------------------------------------
+static void leg_free(TrainState* t) {
+  void* bufs[] = {t->x, t->g[0], t->g[1], t->dlp, t->gcorr, t->ident};
+  for (void* b : bufs) if (b) cudaFree(b);
+  for (int l = 0; l < kMaxLegLayers; ++l) {
+    if (t->act[l]) cudaFree(t->act[l]);
+    t->act[l] = nullptr;
+  }
+  t->x = t->g[0] = t->g[1] = t->dlp = t->gcorr = nullptr;
+  t->ident = nullptr;
+  t->leg_cap = 0;
+}
+
 void train_free(ovn_handle* h) {
   TrainState* t = h->tr;
   if (!t) return;
-  void* bufs[] = {t->o1, t->o2, t->o3, t->dO3, t->dO2, t->dO1, t->corr, t->yaw, t->idx, t->pp, t->ws, t->w3t, t->w2t, t->scale};
+  leg_free(t);
+  void* bufs[] = {t->o1, t->o2, t->o3, t->dO3, t->dO2, t->dO1, t->corr, t->yaw, t->idx, t->pp, t->ws, t->w3t, t->w2t,
+                  t->scale, t->wt};
   for (void* b : bufs) if (b) cudaFree(b);
   for (int l = 0; l < kHeadLayers; ++l) {
     void* lb[] = {t->gk[l], t->gb[l], t->ak[l], t->ab[l]};
+    for (void* b : lb) if (b) cudaFree(b);
+  }
+  for (int l = 0; l < kMaxLegLayers; ++l) {
+    void* lb[] = {t->lgk[l], t->lgb[l], t->lak[l], t->lab[l]};
     for (void* b : lb) if (b) cudaFree(b);
   }
   delete t;
@@ -562,19 +773,17 @@ static int train_alloc(ovn_handle* h) {
   return OVN_OK;
 }
 
-int train_heads_backward(ovn_handle* h, const float* d_bank, int64_t bank_size, const int32_t* d_left,
-                         const int32_t* d_right, int n, const float* d_ov_gt, const int32_t* d_bin_gt,
-                         float min_ov_angle, float* d_losses, cudaStream_t s) {
-  int rc = train_alloc(h);
-  if (rc != OVN_OK) { train_free(h); return rc; }
-  TrainState* t = h->tr;
+// Both heads forward and backward for pairs LEFT = bank[left[p]], RIGHT = bank[right[p]] (bounds-checked
+// indices and yaw bins): losses, the gradients of the four head layers, and dO1 / corr left in t for the
+// feature-volume gradients of ovn_network_backward.
+static int heads_train_core(ovn_handle* h, TrainState* t, const float* d_bank, const int32_t* left,
+                            const int32_t* right, const int32_t* bin, int n, const float* d_ov_gt, float min_ov_angle,
+                            float* d_losses, cudaStream_t s) {
+  int rc = OVN_OK;
   const int Wf = h->cfg.leg_output_width, Cf = kFeatC, sz = h->cfg.conv1size, cap = t->cap;
   const int base = kMaxLegLayers;
   const ConvSpec &L1 = h->head[0], &L2 = h->head[1], &L3 = h->head[2];
   const int n3 = h->dense_in;
-  const int32_t *left = t->idx, *right = t->idx + cap, *bin = t->idx + 2 * cap;
-  k_train_sanitize<<<(n + 255) / 256, 256, 0, s>>>(d_left, d_right, d_bin_gt, n, bank_size, Wf, t->idx, cap, h->d_err);
-  OVN_LAUNCH_CHECK(h);
 
   // ---- forward with saved activations (the launches of heads_forward_fp32)
   {
@@ -657,10 +866,164 @@ int train_heads_backward(ovn_handle* h, const float* d_bank, int64_t bank_size, 
   return OVN_OK;
 }
 
-int train_adagrad_step(ovn_handle* h, float lr, cudaStream_t s) {
+int train_heads_backward(ovn_handle* h, const float* d_bank, int64_t bank_size, const int32_t* d_left,
+                         const int32_t* d_right, int n, const float* d_ov_gt, const int32_t* d_bin_gt,
+                         float min_ov_angle, float* d_losses, cudaStream_t s) {
+  int rc = train_alloc(h);
+  if (rc != OVN_OK) { train_free(h); return rc; }
   TrainState* t = h->tr;
+  const int cap = t->cap;
+  t->have_grad = t->leg_grad = false;
+  k_train_sanitize<<<(n + 255) / 256, 256, 0, s>>>(d_left, d_right, d_bin_gt, n, bank_size, h->cfg.leg_output_width,
+                                                   t->idx, cap, h->d_err);
+  OVN_LAUNCH_CHECK(h);
+  return heads_train_core(h, t, d_bank, t->idx, t->idx + cap, t->idx + 2 * cap, n, d_ov_gt, min_ov_angle, d_losses, s);
+}
+
+// Leg gradients and Adagrad state on the first network call; activation buffers for n pairs (grown, never
+// shrunk, so a training run allocates once).  Handles that only infer or train the heads allocate none of it.
+static int leg_alloc(ovn_handle* h, TrainState* t, int n) {
+  if (!t->leg_alloc) {
+    int64_t kn_max = 0;
+    for (int l = 0; l < h->n_leg; ++l) {
+      const ConvSpec& L = h->leg[l];
+      t->lnk[l] = (int64_t)L.kh * L.kw * L.cin * L.cout;
+      t->lnb[l] = L.cout;
+      if (t->lnk[l] > kn_max) kn_max = t->lnk[l];
+      OVN_CUDA(h, cudaMalloc(&t->lgk[l], t->lnk[l] * sizeof(float)));
+      OVN_CUDA(h, cudaMalloc(&t->lgb[l], t->lnb[l] * sizeof(float)));
+      OVN_CUDA(h, cudaMalloc(&t->lak[l], t->lnk[l] * sizeof(float)));
+      OVN_CUDA(h, cudaMalloc(&t->lab[l], t->lnb[l] * sizeof(float)));
+      const int64_t a = (int64_t)L.h_out * L.w_out * L.cout;
+      if (a > t->max_act) t->max_act = a;
+    }
+    OVN_CUDA(h, cudaMalloc(&t->wt, kn_max * sizeof(float)));
+    if (kn_max * kMaxSplits > t->ws_elems) {
+      cudaFree(t->ws);
+      t->ws = nullptr;
+      t->ws_elems = kn_max * kMaxSplits;
+      OVN_CUDA(h, cudaMalloc(&t->ws, t->ws_elems * sizeof(float)));
+    }
+    t->leg_alloc = true;
+    t->leg_acc_zero = true;
+  }
+  if (n <= t->leg_cap) return OVN_OK;
+  leg_free(t);
+  const int64_t imgs = 2 * (int64_t)n, Wf = h->cfg.leg_output_width;
+  OVN_CUDA(h, cudaMalloc(&t->x, imgs * h->cfg.proj_H * h->cfg.proj_W * h->C * sizeof(float)));
+  for (int l = 0; l < h->n_leg; ++l) {
+    const ConvSpec& L = h->leg[l];
+    OVN_CUDA(h, cudaMalloc(&t->act[l], imgs * L.h_out * L.w_out * L.cout * sizeof(float)));
+  }
+  OVN_CUDA(h, cudaMalloc(&t->g[0], imgs * t->max_act * sizeof(float)));
+  OVN_CUDA(h, cudaMalloc(&t->g[1], imgs * t->max_act * sizeof(float)));
+  OVN_CUDA(h, cudaMalloc(&t->dlp, (int64_t)n * h->o1_w * Wf * kFeatC * sizeof(float)));
+  OVN_CUDA(h, cudaMalloc(&t->gcorr, (int64_t)n * Wf * sizeof(float)));
+  OVN_CUDA(h, cudaMalloc(&t->ident, 2 * (int64_t)n * sizeof(int32_t)));
+  t->leg_cap = n;
+  return OVN_OK;
+}
+
+int train_network_backward(ovn_handle* h, const float* d_inputs, int64_t n_inputs, const int32_t* d_left,
+                           const int32_t* d_right, const int32_t* d_roll, int n, const float* d_ov_gt,
+                           const int32_t* d_bin_gt, float min_ov_angle, float* d_losses, cudaStream_t s) {
+  if (h->cfg.conv1size > 256 / kDfvC)
+    OVN_SET_ERR(h, OVN_ERR_BAD_CONFIG, "ovn_network_backward: conv1size %d > %d is not supported", h->cfg.conv1size,
+                256 / kDfvC);
+  int rc = train_alloc(h);
+  if (rc != OVN_OK) { train_free(h); return rc; }
+  TrainState* t = h->tr;
+  rc = leg_alloc(h, t, n);
+  if (rc != OVN_OK) { train_free(h); return rc; }
+  const int cap = t->cap, Wf = h->cfg.leg_output_width, sz = h->cfg.conv1size, nb = h->o1_w;
+  const int H = h->cfg.proj_H, W = h->cfg.proj_W, C = h->C, last = h->n_leg - 1;
+  t->have_grad = t->leg_grad = false;
+  k_train_sanitize<<<(n + 255) / 256, 256, 0, s>>>(d_left, d_right, d_bin_gt, n, n_inputs, Wf, t->idx, cap, h->d_err);
+  OVN_LAUNCH_CHECK(h);
+
+  // ---- leg forward over the 2n gathered images, every activation kept (the launches of leg_forward_fp32)
+  {
+    const int64_t e = 2 * (int64_t)n * H * W * C;
+    k_gather_inputs<<<(unsigned)((e + 255) / 256), 256, 0, s>>>(d_inputs, t->idx, t->idx + cap, d_roll, n, H, W, C,
+                                                                t->x);
+    OVN_LAUNCH_CHECK(h);
+  }
+  // The leg GEMMs run over at most kLegImgChunk images per launch (the grid's y extent is bounded); an
+  // output's arithmetic does not depend on M, so the chunking changes no bit.
+  const float* x = t->x;
+  for (int l = 0; l <= last; ++l) {
+    const ConvSpec& L = h->leg[l];
+    const int64_t in_img = (int64_t)L.h_in * L.w_in * L.cin, out_img = (int64_t)L.h_out * L.w_out * L.cout;
+    for (int i0 = 0; i0 < 2 * n; i0 += kLegImgChunk) {
+      const int ni = 2 * n - i0 < kLegImgChunk ? 2 * n - i0 : kLegImgChunk;
+      ConvOperand a{x + i0 * in_img, L.h_in, L.w_in, L.cin, L.kw, L.sh, L.sw, L.h_out, L.w_out};
+      BOperand b{h->d_w[l], nullptr, nullptr, 0, 0};
+      rc = launch_gemm(h, a, b, h->d_b[l], t->act[l] + i0 * out_img, ni * L.h_out * L.w_out, L.cout,
+                       L.kh * L.kw * L.cin, 1, L.relu, s);
+      if (rc != OVN_OK) return rc;
+    }
+    x = t->act[l];
+  }
+  const float* fv = t->act[last];
+
+  // ---- both heads on the trained volumes, LEFT = p, RIGHT = n + p
+  k_pair_ident<<<(n + 255) / 256, 256, 0, s>>>(t->ident, n, n);
+  OVN_LAUNCH_CHECK(h);
+  const int32_t* bin = t->idx + 2 * cap;
+  rc = heads_train_core(h, t, fv, t->ident, t->ident + n, bin, n, d_ov_gt, min_ov_angle, d_losses, s);
+  if (rc != OVN_OK) return rc;
+  t->have_grad = false;
+
+  // ---- dFV = overlap-head part + correlation-head part, masked by the ReLU of s_conv10
+  float* dfv = t->g[0];
+  k_corr_logit_grad<<<n, 128, 0, s>>>(t->corr, d_ov_gt, bin, min_ov_angle, n, Wf, t->gcorr);
+  OVN_LAUNCH_CHECK(h);
+  k_dfv_overlap<<<dim3(kFeatC / kDfvC, nb, n), 256, 0, s>>>(fv, t->dO1, h->d_w[kMaxLegLayers], n, Wf, sz, nb, t->dlp,
+                                                            dfv);
+  OVN_LAUNCH_CHECK(h);
+  k_dfv_finish<<<dim3((Wf + kFinRows - 1) / kFinRows, 2, n), 128, Wf * sizeof(float), s>>>(fv, t->gcorr, t->dlp, n, Wf,
+                                                                                          nb, dfv);
+  OVN_LAUNCH_CHECK(h);
+
+  // ---- leg backward, s_conv10 .. s_conv1: dW, db over all 2n images; dX (strided) for every layer but the first
+  float* dY = dfv;
+  for (int l = last; l >= 0; --l) {
+    const ConvSpec& L = h->leg[l];
+    const float* X = l > 0 ? t->act[l - 1] : t->x;
+    const int M = 2 * n * L.h_out * L.w_out, K = L.kh * L.kw * L.cin;
+    ConvOperand a{X, L.h_in, L.w_in, L.cin, L.kw, L.sh, L.sw, L.h_out, L.w_out};
+    rc = weight_grad(h, t, a, dY, M, K, L.cout, t->lgk[l], s);
+    if (rc == OVN_OK) rc = bias_grad(h, t, dY, M, L.cout, t->lgb[l], s);
+    if (rc != OVN_OK) return rc;
+    if (l == 0) break;
+    k_transpose_taps<<<(unsigned)((t->lnk[l] + 255) / 256), 256, 0, s>>>(h->d_w[l], L.kh * L.kw, L.cin, L.cout, t->wt);
+    OVN_LAUNCH_CHECK(h);
+    float* dX = dY == t->g[0] ? t->g[1] : t->g[0];
+    const int64_t in_img = (int64_t)L.h_in * L.w_in * L.cin, out_img = (int64_t)L.h_out * L.w_out * L.cout;
+    for (int i0 = 0; i0 < 2 * n; i0 += kLegImgChunk) {
+      const int ni = 2 * n - i0 < kLegImgChunk ? 2 * n - i0 : kLegImgChunk;
+      ConvTOperand at{dY + i0 * out_img, L.h_in, L.w_in, L.h_out, L.w_out, L.kw, L.cout, L.sh, L.sw};
+      BOperand bt{t->wt, nullptr, nullptr, 0, 0};
+      rc = launch_gemm(h, at, bt, nullptr, dX + i0 * in_img, ni * L.h_in * L.w_in, L.cin, L.kh * L.kw * L.cout, 1, 0, s);
+      if (rc != OVN_OK) return rc;
+    }
+    const int64_t nx = 2 * n * in_img;
+    k_relu_mask<<<(unsigned)((nx + 255) / 256), 256, 0, s>>>(dX, t->act[l - 1], nx);
+    OVN_LAUNCH_CHECK(h);
+    dY = dX;
+  }
+  t->have_grad = t->leg_grad = true;
+  return OVN_OK;
+}
+
+// Updates the layers the last backward call produced gradients for: the four head layers, plus the leg
+// after ovn_network_backward.  *leg_changed tells the caller whether the leg weights moved.
+int train_adagrad_step(ovn_handle* h, float lr, cudaStream_t s, bool* leg_changed) {
+  TrainState* t = h->tr;
+  *leg_changed = false;
   if (!t || !t->have_grad)
-    OVN_SET_ERR(h, OVN_ERR_INVALID_ARG, "ovn_adagrad_step: no gradients yet (call ovn_heads_backward first)");
+    OVN_SET_ERR(h, OVN_ERR_INVALID_ARG,
+                "ovn_adagrad_step: no gradients yet (call ovn_heads_backward or ovn_network_backward first)");
   if (t->acc_zero) {
     for (int l = 0; l < kHeadLayers; ++l) {
       OVN_CUDA(h, cudaMemsetAsync(t->ak[l], 0, t->nk[l] * sizeof(float), s));
@@ -675,20 +1038,44 @@ int train_adagrad_step(ovn_handle* h, float lr, cudaStream_t s) {
     k_adagrad<<<(unsigned)((t->nb[l] + 255) / 256), 256, 0, s>>>(h->d_b[slot], t->gb[l], t->ab[l], t->nb[l], lr);
     OVN_LAUNCH_CHECK(h);
   }
+  if (!t->leg_grad) return OVN_OK;
+  if (t->leg_acc_zero) {
+    for (int l = 0; l < h->n_leg; ++l) {
+      OVN_CUDA(h, cudaMemsetAsync(t->lak[l], 0, t->lnk[l] * sizeof(float), s));
+      OVN_CUDA(h, cudaMemsetAsync(t->lab[l], 0, t->lnb[l] * sizeof(float), s));
+    }
+    t->leg_acc_zero = false;
+  }
+  for (int l = 0; l < h->n_leg; ++l) {
+    k_adagrad<<<(unsigned)((t->lnk[l] + 255) / 256), 256, 0, s>>>(h->d_w[l], t->lgk[l], t->lak[l], t->lnk[l], lr);
+    OVN_LAUNCH_CHECK(h);
+    k_adagrad<<<(unsigned)((t->lnb[l] + 255) / 256), 256, 0, s>>>(h->d_b[l], t->lgb[l], t->lab[l], t->lnb[l], lr);
+    OVN_LAUNCH_CHECK(h);
+  }
+  *leg_changed = true;
   return OVN_OK;
 }
 
 void train_reset_optimizer(ovn_handle* h) {
-  if (h->tr) h->tr->acc_zero = true;
+  if (h->tr) h->tr->acc_zero = h->tr->leg_acc_zero = true;
 }
 
+bool train_has_leg_gradients(const ovn_handle* h) { return h->tr && h->tr->have_grad && h->tr->leg_grad; }
+
+// layer: 0..3 = c_conv1..3, overlap_output; kMaxLegLayers + l = leg layer l (after ovn_network_backward only)
 int train_get_gradient(ovn_handle* h, int layer, float* h_kernel, float* h_bias) {
   TrainState* t = h->tr;
   if (!t || !t->have_grad)
-    OVN_SET_ERR(h, OVN_ERR_INVALID_ARG, "ovn_get_gradient: no gradients yet (call ovn_heads_backward first)");
+    OVN_SET_ERR(h, OVN_ERR_INVALID_ARG,
+                "ovn_get_gradient: no gradients yet (call ovn_heads_backward or ovn_network_backward first)");
+  const bool leg = layer >= kMaxLegLayers;
+  const int l = leg ? layer - kMaxLegLayers : layer;
+  const float* gk = leg ? t->lgk[l] : t->gk[l];
+  const float* gb = leg ? t->lgb[l] : t->gb[l];
+  const int64_t nk = leg ? t->lnk[l] : t->nk[l], nb = leg ? t->lnb[l] : t->nb[l];
   OVN_CUDA(h, cudaEventSynchronize(h->ev_train));
-  if (h_kernel) OVN_CUDA(h, cudaMemcpy(h_kernel, t->gk[layer], t->nk[layer] * sizeof(float), cudaMemcpyDeviceToHost));
-  if (h_bias) OVN_CUDA(h, cudaMemcpy(h_bias, t->gb[layer], t->nb[layer] * sizeof(float), cudaMemcpyDeviceToHost));
+  if (h_kernel) OVN_CUDA(h, cudaMemcpy(h_kernel, gk, nk * sizeof(float), cudaMemcpyDeviceToHost));
+  if (h_bias) OVN_CUDA(h, cudaMemcpy(h_bias, gb, nb * sizeof(float), cudaMemcpyDeviceToHost));
   return OVN_OK;
 }
 

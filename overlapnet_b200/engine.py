@@ -306,7 +306,7 @@ class Engine:
   def bank_release(self, bank=None):
     check(self._h, lib().ovn_bank_release(self._h, _ptr(bank)), 'ovn_bank_release')
 
-  # ---- overlap-head training on a frozen leg (precision fp32) ---------------------------------
+  # ---- training: the overlap head on a frozen leg, or the full network -------------------------
   HEAD_LAYERS = ('c_conv1', 'c_conv2', 'c_conv3', 'overlap_output')
 
   def heads_backward(self, bank, left_idx, right_idx, overlap_gt, yaw_bin_gt, min_overlap_for_angle=0.7):
@@ -323,6 +323,28 @@ class Engine:
     check(self._h, lib().ovn_heads_backward(self._h, _ptr(bank), int(bank.shape[0]), _ptr(li), _ptr(ri), n, _ptr(ov),
                                            _ptr(yb), float(min_overlap_for_angle), _ptr(losses), self._stream()),
           'ovn_heads_backward')
+    self._leg_grads = False
+    return losses
+
+  def network_backward(self, inputs, left_idx, right_idx, overlap_gt, yaw_bin_gt, right_roll=None,
+                       min_overlap_for_angle=0.7):
+    """ovn_network_backward: losses and the gradients of every layer for pairs LEFT = inputs[left_idx],
+    RIGHT = inputs[right_idx] rolled by ``right_roll`` columns (np.roll along the width; None = no roll).
+    ``inputs``: packed network inputs [n, H, W, C] float32 cuda.  Returns the losses like
+    ``heads_backward``; the gradients stay in the handle (``gradients()``, ``adagrad_step``)."""
+    n = left_idx.numel()
+    dev = self.device
+    x = inputs.to(device=dev, dtype=torch.float32).contiguous()
+    li = left_idx.to(device=dev, dtype=torch.int32).contiguous()
+    ri = right_idx.to(device=dev, dtype=torch.int32).contiguous()
+    ro = None if right_roll is None else torch.as_tensor(right_roll).to(device=dev, dtype=torch.int32).contiguous()
+    ov = torch.as_tensor(overlap_gt).to(device=dev, dtype=torch.float32).contiguous()
+    yb = torch.as_tensor(yaw_bin_gt).to(device=dev, dtype=torch.int32).contiguous()
+    losses = torch.empty((3,), dtype=torch.float32, device=dev)
+    check(self._h, lib().ovn_network_backward(self._h, _ptr(x), int(x.shape[0]), _ptr(li), _ptr(ri), _ptr(ro), n,
+                                             _ptr(ov), _ptr(yb), float(min_overlap_for_angle), _ptr(losses),
+                                             self._stream()), 'ovn_network_backward')
+    self._leg_grads = True
     return losses
 
   def _layer_arrays(self, fn, what, names=None):
@@ -338,8 +360,10 @@ class Engine:
     return out
 
   def gradients(self):
-    """{layer: (kernel grad, bias grad)} of the head layers after the last ``heads_backward``, keyed
-    like ``weights.glorot_init``; synchronises."""
+    """{layer: (kernel grad, bias grad)} keyed like ``weights.glorot_init``: every layer after a
+    ``network_backward``, the head layers after a ``heads_backward``; synchronises."""
+    if getattr(self, '_leg_grads', False):
+      return self._layer_arrays(lib().ovn_get_gradient, 'ovn_get_gradient')
     return self._layer_arrays(lib().ovn_get_gradient, 'ovn_get_gradient', self.HEAD_LAYERS)
 
   def get_weights(self):
