@@ -145,6 +145,22 @@ int ovn_gt_overlap_count(ovn_handle* h, const float* d_ref_ranges /* [n][H][W] *
                          const float* d_cur_range /* [H][W] */, int32_t n_scans,
                          int32_t* d_counts /* [n_scans + 1] */, void* stream);
 
+/* For pair k (d_pairs[2k] = current frame c, d_pairs[2k+1] = reference scan r):
+ * d_counts[k] = #{pixels: ref > 0 and |ref - cur_c| < 1}, where ref = scan r moved by d_pose_ref[r]
+ * and then d_pose_cur_inv[c] (float64), projected as in ovn_gt_range_batch.  Equal to
+ * ovn_gt_range_batch + ovn_gt_overlap_count of that pair.  com_overlap_yaw.py:35-46 for many frames.
+ * Scan r is d_points[d_offsets[r] .. d_offsets[r+1]); d_cur_ranges are the current frames' images as
+ * ovn_gt_range_batch makes them without poses.  One CTA builds each pair's H x W image in shared
+ * memory: OVN_ERR_BAD_CONFIG when H*W*4 bytes exceed what a block may use (64 x 900 fits).  Order
+ * the pairs reference-major so that concurrent CTAs share one scan's points in L2.  Indices outside
+ * [0, n_cur) / [0, n_scans) are clamped, the count is poisoned (-1) and the next synchronising call
+ * (ovn_check) returns OVN_ERR_INVALID_ARG.  max_range < 0 selects the handle's configured max_range. */
+int ovn_gt_pair_counts(ovn_handle* h, const float* d_points, const int64_t* d_offsets, int32_t n_scans,
+                       int64_t n_points_total, const double* d_pose_ref /* [n_scans][16] */,
+                       const double* d_pose_cur_inv /* [n_cur][16] */, const float* d_cur_ranges /* [n_cur][H][W] */,
+                       int32_t n_cur, const int32_t* d_pairs /* [n_pairs][2] */, int64_t n_pairs,
+                       float max_range, int32_t* d_counts /* [n_pairs] */, void* stream);
+
 /* ---- stage 1d: fused raw cloud -> packed network input ------------------------------------- */
 /* Projection + normals + channel packing (ImagePairOverlapOrientationSequence.py:130-207) in one
  * pass; d_probs may be NULL when n_prob_channels == 0.  d_input: [n][H][W][C] float32. */

@@ -21,7 +21,7 @@ SYMBOLS = [
     'ovn_query_cloud_vs_bank_host', 'ovn_check', 'ovn_set_feature_center', 'ovn_get_feature_center',
     'ovn_heads_rows_vs_bank', 'ovn_calibrate', 'ovn_peer_signal', 'ovn_peer_wait',
     'ovn_heads_backward', 'ovn_get_gradient', 'ovn_adagrad_step', 'ovn_get_weights',
-    'ovn_network_backward',
+    'ovn_network_backward', 'ovn_gt_pair_counts',
 ]
 
 
@@ -79,6 +79,7 @@ def lib():
   L.ovn_normals_batch.argtypes = [vp, vp, vp, i32, vp, vp]
   L.ovn_gt_range_batch.argtypes = [vp, vp, vp, i32, i64, vp, vp, f32, vp, vp]
   L.ovn_gt_overlap_count.argtypes = [vp, vp, vp, i32, vp, vp]
+  L.ovn_gt_pair_counts.argtypes = [vp, vp, vp, i32, i64, vp, vp, vp, i32, vp, i64, f32, vp, vp]
   L.ovn_semantic_batch.argtypes = [vp, vp, vp, vp, i32, i32, vp, vp]
   L.ovn_preprocess_batch.argtypes = [vp, vp, vp, i32, i64, vp, vp, vp]
   L.ovn_pack_input.argtypes = [vp, vp, vp, vp, vp, i32, vp, vp]

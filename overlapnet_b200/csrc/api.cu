@@ -480,6 +480,21 @@ int ovn_gt_overlap_count(ovn_handle* h, const float* d_ref_ranges, const float* 
   return gt_overlap_count(h, d_ref_ranges, d_cur_range, n_scans, d_counts, (cudaStream_t)stream);
 }
 
+int ovn_gt_pair_counts(ovn_handle* h, const float* d_points, const int64_t* d_offsets, int32_t n_scans,
+                       int64_t n_points_total, const double* d_pose_ref, const double* d_pose_cur_inv,
+                       const float* d_cur_ranges, int32_t n_cur, const int32_t* d_pairs, int64_t n_pairs,
+                       float max_range, int32_t* d_counts, void* stream) {
+  if (!h) return OVN_ERR_INVALID_ARG;
+  DeviceGuard guard(h);
+  REQUIRE(h, n_pairs >= 0 && n_points_total >= 0, "negative size");
+  if (n_pairs == 0) return OVN_OK;
+  REQUIRE(h, n_scans > 0 && n_cur > 0, "n_scans and n_cur must be positive");
+  REQUIRE(h, d_offsets && d_pose_ref && d_pose_cur_inv && d_cur_ranges && d_pairs && d_counts &&
+                 (d_points || n_points_total == 0), "NULL pointer");
+  return gt_pair_counts(h, d_points, d_offsets, n_scans, n_points_total, d_pose_ref, d_pose_cur_inv, d_cur_ranges,
+                        n_cur, d_pairs, n_pairs, max_range, d_counts, (cudaStream_t)stream);
+}
+
 int ovn_preprocess_batch(ovn_handle* h, const float* d_points, const int64_t* d_offsets, int32_t n_scans,
                          int64_t n_total, const float* d_probs, float* d_input, void* stream) {
   if (!h) return OVN_ERR_INVALID_ARG;

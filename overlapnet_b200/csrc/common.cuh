@@ -164,6 +164,9 @@ int gt_range_batch(ovn_handle* h, const float* d_points, const int64_t* d_offset
                    const double* d_pose_ref, const double* d_pose_cur_inv, float max_range, float* d_range,
                    cudaStream_t s);
 int gt_overlap_count(ovn_handle* h, const float* d_ref, const float* d_cur, int n_scans, int32_t* d_counts, cudaStream_t s);
+int gt_pair_counts(ovn_handle* h, const float* d_points, const int64_t* d_offsets, int n_scans, int64_t n_total,
+                   const double* d_pose_ref, const double* d_pose_cur_inv, const float* d_cur, int n_cur,
+                   const int32_t* d_pairs, int64_t n_pairs, float max_range, int32_t* d_counts, cudaStream_t s);
 int pack_input(ovn_handle* h, const float* d_depth, const float* d_normal, const float* d_prob,
                const float* d_intensity, int n_scans, float* d_input, cudaStream_t s);
 

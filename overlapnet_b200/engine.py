@@ -208,6 +208,27 @@ class Engine:
                                              self._stream()), 'ovn_gt_overlap_count')
     return counts
 
+  def gt_pair_counts(self, batch, pose_ref, pose_cur_inv, cur_ranges, pairs, max_range=-1.0, out=None):
+    """ovn_gt_pair_counts: int32 [n_pairs]; for pair k = (current c, reference r) = ``pairs[k]`` the
+    ``gt_overlap_count`` of scan r of ``batch`` moved by ``pose_ref[r]`` and then ``pose_cur_inv[c]``
+    against ``cur_ranges[c]``, without materialising the reference image.  ``pose_ref``: (n, 4, 4) and
+    ``pose_cur_inv``: (n_cur, 4, 4) float64; ``cur_ranges``: [n_cur, H, W] float32 cuda (``gt_range``
+    with no poses); ``pairs``: [n_pairs, 2] int32, best reference-major.  ``out``: int32 cuda tensor to
+    write into.  Out-of-range indices give -1 and an error at the next ``check``."""
+    dev = self.device
+    pr = torch.as_tensor(pose_ref, dtype=torch.float64).reshape(batch.n, 16).to(dev).contiguous()
+    pc = torch.as_tensor(pose_cur_inv, dtype=torch.float64).reshape(-1, 16).to(dev).contiguous()
+    cur = cur_ranges.to(device=dev, dtype=torch.float32).contiguous()
+    pl = torch.as_tensor(pairs).to(device=dev, dtype=torch.int32).reshape(-1, 2).contiguous()
+    n_pairs = pl.shape[0]
+    counts = out if out is not None else torch.empty((n_pairs,), dtype=torch.int32, device=dev)
+    assert counts.dtype == torch.int32 and counts.is_contiguous() and counts.numel() == n_pairs
+    check(self._h, lib().ovn_gt_pair_counts(
+        self._h, _ptr(batch.points), _ptr(batch.offsets), batch.n, int(batch.points.shape[0]), _ptr(pr), _ptr(pc),
+        _ptr(cur), int(cur.shape[0]), _ptr(pl), n_pairs, float(max_range), _ptr(counts), self._stream()),
+        'ovn_gt_pair_counts')
+    return counts
+
   def normals(self, rng, vertex):
     n = rng.shape[0]
     out = torch.empty((n, self.H, self.W, 3), dtype=torch.float32, device=self.device)
